@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BBBAlexNet forward + KL images/sec on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--dump-outputs DIR] [--impl reference]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one synthetic batch: BBBAlexNet
@@ -10,7 +10,10 @@ all six Bayesian layers + the model file's own activation/pool/flatten modules +
 the summed KL scalar.  With N GPUs the num_ens MC loop (main_bayesian.py:46-49)
 is the shard axis: rank r runs sample r of the SAME batch and one NCCL all-reduce
 combines sum_j softmax_j and the KL (SURVEY.md 8e) -> weak scaling, value =
-B * N * K / t.
+B * N * K / t.  The value times exactly K steps, in one window after the W warm-up
+steps (before those, every captured graph is replayed once, untimed: a graph's first
+replay uploads it).  Inputs, parameters and noise seeds are fixed, so with the same arguments
+--dump-outputs writes the same step outputs (log_outputs, kl, ...) on every run.
 
 Printed JSON (rank 0, one line): the driver contract + `roofline`, `cpu_baseline`,
 `e2e`, `clocks`, `gpu_launches`, `per_layer`.
@@ -19,6 +22,7 @@ from __future__ import annotations
 
 import argparse
 import json
+import math
 import os
 import statistics
 import subprocess
@@ -225,7 +229,8 @@ def run_ours(args):
     n_inputs = 4                                 # pinned host batches (e2e arm)
     n_dev_inputs = max(2, -(-(160 << 20) // in_bytes))   # device-resident arm rotates through > 126 MB (L2) of inputs
     x_host = [torch.randn(*in_shape, generator=gx).pin_memory() for _ in range(n_inputs)]
-    x_dev = [torch.randn(*in_shape, device=dev) for _ in range(n_dev_inputs)]
+    gd = torch.Generator(device=dev).manual_seed(123)    # seeded: the same arguments give the same inputs on every run
+    x_dev = [torch.randn(*in_shape, device=dev, generator=gd) for _ in range(n_dev_inputs)]
     # The step = the package's public MC step (mc.MCForward): this rank's samples through the engine (fused tcgen05 chain),
     # then ONE kernel that combines them, exchanges the partials with the other ranks over NVLink and finishes
     # logmeanexp / KL (/ uncertainty) on the device -- all in one captured CUDA graph per resident input batch.
@@ -237,7 +242,7 @@ def run_ours(args):
     # are bit-identical to the serial engine (tests/test_gpu_mc.py).  The one-step-at-a-time figure is under serial_step.
     infl = int(os.environ.get("BBB_B200_MC_INFLIGHT", "4")) if ovl else 1
     eng = mc.MCForward(net, x_dev[0], S_total, want_uncertainty=cfg["uncertainty"], seed=2024, static_inputs=x_dev, overlap=ovl, inflight=infl)
-    staging = [torch.empty_like(x_dev[0]) for _ in range(2)]
+    staging = [torch.zeros_like(x_dev[0]) for _ in range(2)]
     eng_e2e = mc.MCForward(net, x_dev[0], S_total, want_uncertainty=cfg["uncertainty"], seed=2024, static_inputs=staging,
                            first_replay=1 << 18, overlap=ovl, inflight=infl)
     S_local = len(eng.ids)
@@ -262,6 +267,14 @@ def run_ours(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
+    def prime(engine, slots):
+        """Replay every graph the engine captured once, untimed: a graph's first replay uploads it to the device.  Steps
+        cycle through the (in-flight buffer, input slot) pairs with period lcm(nbuf, slots)."""
+        for i in range(math.lcm(engine.nbuf, slots)):
+            engine(slot=i % slots)
+        engine.wait()
+        sync_all()
+
     # ---- device-resident throughput: K steps back to back, inputs rotate through > L2 of resident batches ----
     counter = [0]
 
@@ -271,14 +284,15 @@ def run_ours(args):
             counter[0] += 1
         eng.wait()
 
+    prime(eng, n_dev_inputs)
     window(resident, args.warmup)
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     wall0 = time.perf_counter()
-    wins = [window(resident, args.steps) for _ in range(args.windows)]
+    total_ms = window(resident, args.steps)
     wall = time.perf_counter() - wall0
-    total_ms = statistics.median(wins)
+    last_step = {k: v.cpu() for k, v in eng.out.items()} if args.dump_outputs and rank == 0 else None
     images_per_step = B * S_total                # image-samples of the whole job per step (SURVEY 8d: B*S/t)
     value = images_per_step * args.steps / (total_ms * 1e-3)
     launches = eng.kernels_per_step * args.steps
@@ -315,9 +329,9 @@ def run_ours(args):
         if eng_e2e.result_stream is not None:
             main.wait_stream(eng_e2e.result_stream)
 
+    prime(eng_e2e, len(staging))
     window(e2e_steps, max(3, args.warmup))
-    e2e_wins = [window(e2e_steps, args.steps) for _ in range(max(5, args.windows // 3))]
-    e2e_ms = statistics.median(e2e_wins)
+    e2e_ms = window(e2e_steps, args.steps)
     e2e_value = images_per_step * args.steps / (e2e_ms * 1e-3)
     clocks = sampler.stop() if rank == 0 else None
     timeouts = eng.timeouts() + eng_e2e.timeouts()
@@ -332,9 +346,9 @@ def run_ours(args):
                 eng_s(slot=counter[0] % n_dev_inputs)
                 counter[0] += 1
 
+        prime(eng_s, n_dev_inputs)
         window(resident_serial, args.warmup)
-        s_wins = [window(resident_serial, args.steps) for _ in range(max(5, args.windows // 3))]
-        s_ms = statistics.median(s_wins)
+        s_ms = window(resident_serial, args.steps)
         serial = {"ms_per_step": s_ms / args.steps, "value": images_per_step * args.steps / (s_ms * 1e-3), "unit": "images/s",
                   "note": "one step in flight, exchange kernel inside the step's graph (the step latency); the headline value "
                           f"keeps {infl} independent steps in flight"}
@@ -454,12 +468,9 @@ def run_ours(args):
                                   "exchange kernel over NVLink peer memory on its own stream, beside the next step's chain)" if ovl else
                                   "one CUDA graph replay per step (noise advance, per-layer prep + GEMM kernels, MC exchange kernel over "
                                   "NVLink peer memory)") + "; one captured graph per resident input batch, read in place",
-                       "timing": f"median of {args.windows} windows of {args.steps} steps, each bracketed by barrier+synchronize, "
-                                 f"CUDA events, max over ranks per window"},
-            "windows_ms": {"min": min(wins), "median": total_ms, "max": max(wins), "n": len(wins)},
+                       "timing": f"{args.steps} steps in one window bracketed by barrier+synchronize, CUDA events, max over ranks"},
             "e2e": {"value": e2e_value, "unit": "images/s", "h2d_bytes_per_step": in_bytes,
-                    "d2h_bytes_per_step": B * C * 4 + 4, "windows_ms": {"min": min(e2e_wins), "median": e2e_ms, "max": max(e2e_wins)},
-                    "host_numa": numa},
+                    "d2h_bytes_per_step": B * C * 4 + 4, "ms_per_step": e2e_ms / args.steps, "host_numa": numa},
             "gpu_launches": int(launches),
             "serial_step": serial,
             "clocks": clocks,
@@ -474,10 +485,32 @@ def run_ours(args):
             "wall_s_timed_loop": wall,
         }
         print(json.dumps(out), flush=True)
+        if last_step is not None:
+            dump_outputs(last_step, args.dump_outputs)
     sync_all()
     eng.close(); eng_e2e.close()
     if dist is not None:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out, path):
+    """Write each output of the step as <path>/<name>.npy (float32).  Above DUMP_BYTES in all, every [B, ...] output keeps
+    the same fixed, seeded sample of batch rows, so that two builds run with the same arguments compare row for row."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    total = sum(v.numel() * 4 for v in out.values())
+    rows = None
+    if total > DUMP_BYTES:
+        B = next(v.shape[0] for v in out.values() if v.dim() > 0)
+        keep = max(1, B * DUMP_BYTES // total)
+        rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    for name, v in out.items():
+        if rows is not None and v.dim() > 0:
+            v = v[rows]
+        np.save(os.path.join(path, f"{name}.npy"), v.float().numpy())
 
 
 def in_chain_kernels(net, x, dev, reps=20):
@@ -746,7 +779,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--mc-batch", type=int, default=10, help="also report S MC samples folded into one launch (LRT; 0 = skip)")
     ap.add_argument("--train-steps", type=int, default=5, help="steps per window of the sharded training-step figure (0 = skip)")
-    ap.add_argument("--windows", type=int, default=25, help="timed windows of --steps steps; the median window is reported")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed step returned in its last step as DIR/<name>.npy (float32, at most 64 MB)")
     ap.add_argument("--config", default="headline", choices=list(CONFIGS),
                     help="headline (default: BBBAlexNet-10 B=512, one MC sample per GPU per step) or one of BASELINE.json's configs restated")
     args = ap.parse_args()

@@ -3,7 +3,7 @@
 The reference's model files (models/BayesianModels/BayesianAlexNet.py:8-53,
 BayesianLeNet.py:8-49, Bayesian3Conv3FC.py:7-55) are constructor-only and run
 UNCHANGED on top of this repo's ``layers`` package (tests/test_dropin.py checks
-that where /root/reference exists).  They cannot travel to the GPU box, so the
+these tables against what those files build).  The package does not ship them, so the
 benchmark and GPU tests build the same networks from the tables below: same
 child names in the same order (=> same state_dict keys, same ModuleWrapper
 iteration order), same constructor signature.

@@ -25,8 +25,16 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def golden_layers():
+    """The layer cases of every layers_<kind>_<variant>.npz, as one mapping."""
+    import glob
     import numpy as np
-    return np.load(os.path.join(GOLDEN, "layers.npz"))
+    parts = sorted(glob.glob(os.path.join(GOLDEN, "layers_*.npz")))
+    assert parts, "tests/golden/layers_*.npz missing"
+    out = {}
+    for p in parts:
+        with np.load(p) as z:
+            out.update({k: z[k] for k in z.files})
+    return out
 
 
 @pytest.fixture(scope="session")

@@ -1,24 +1,35 @@
-"""Generate golden fixtures by running the UNMODIFIED reference in this container.
+"""Generate golden fixtures by running the UNMODIFIED reference project.
 
-    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
+    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py <PyTorch-BayesianCNN checkout>
 
-Imports /root/reference (read-only) -- never copied into the repo -- runs its
-layers / models on seeded inputs, recovers the eps it drew by seed-replay of the
-global CPU generator (SURVEY.md 8c), and writes small ``.npz`` files next to
-this script.  /root/reference does not exist on the GPU box, so nothing in the
-test-suite calls this script; it is committed so the fixtures are reproducible.
+Imports the reference checkout given on the command line (read-only, never
+copied into this repo), runs its layers / models on seeded inputs, recovers the
+eps it drew by seed-replay of the global CPU generator (SURVEY.md 8c), and
+writes small files next to this script.  The test-suite only reads the fixtures;
+this script is committed so they are reproducible.
 
-Fixtures
-  layers.npz  : per-layer cases (x, params, eps, y, kl) for conv/linear x bbb/lrt
+Fixtures (each file stays below 1 MB)
+  layers_<kind>_<variant>.npz : per-layer cases (x, params, eps, y, kl) for
+                conv/lin x bbb/lrt
   models.npz  : the three model files, both variants: x, logits, kl, and float64
                 checksums of every parameter (params are re-drawn from the seed
                 by oracle.init_params; the checksums prove the re-draw matches)
+  dropin.json : what the model files need from the ``layers`` package (the names
+                they import, their child list as ``layers`` exports / torch.nn
+                types, state_dict keys and shapes), for the drop-in tests
+  dropin.npz  : BBBLeNet, bbb layers, relu -- the one activation / variant pair of
+                LeNet that models.npz lacks: x, logits, kl, parameter checksums
 """
+import ast
+import glob
+import json
 import os
 import sys
 
 sys.dont_write_bytecode = True
-REF = "/root/reference"
+if len(sys.argv) != 2:
+    raise SystemExit(__doc__)
+REF = os.path.abspath(sys.argv[1])
 HERE = os.path.dirname(os.path.abspath(__file__))
 # the reference's layer files do `sys.path.append("..")` and import top-level
 # `metrics`; run with the reference root first on sys.path, like `cd reference`.
@@ -144,17 +155,57 @@ def model_case(name, cls, key, inputs, outputs, variant, act, batch, out):
     out[pre + "param_names"] = np.array([n for n, _ in net.named_parameters()])
 
 
+def layers_export(m):
+    """The name under which the reference's ``layers`` package exports type(m), else the torch.nn type name."""
+    for name in ref_layers.__all__ if hasattr(ref_layers, "__all__") else dir(ref_layers):
+        if type(m) is getattr(ref_layers, name):
+            return "layers." + name
+    return "nn." + type(m).__name__
+
+
+def dropin_structure():
+    imports = set()
+    for f in sorted(glob.glob(os.path.join(REF, "models", "BayesianModels", "*.py"))):
+        for node in ast.walk(ast.parse(open(f).read())):
+            if isinstance(node, ast.ImportFrom) and node.module == "layers":
+                imports.update(a.name for a in node.names)
+    nets = {}
+    for cls, key, inputs in ((BBBAlexNet, "alexnet", 3), (BBBLeNet, "lenet", 3), (BBB3Conv3FC, "3conv3fc", 1)):
+        for variant in ("lrt", "bbb"):
+            net = cls(10, inputs, CFG_PRIORS, variant, "softplus")
+            assert isinstance(net, ref_layers.ModuleWrapper)
+            nets[f"{key}_{variant}"] = {
+                "class": cls.__name__, "inputs": inputs, "variant": variant,
+                "children": [f"{n} {layers_export(m)}" for n, m in net.named_children()],
+                "state_dict": [f"{k} {'x'.join(map(str, v.shape))}" for k, v in net.state_dict().items()]}
+        for bad in (dict(layer_type="nope"), dict(activation_type="nope")):
+            try:
+                cls(10, inputs, CFG_PRIORS, **bad)
+            except ValueError:
+                continue
+            raise AssertionError(f"{cls.__name__}({bad}) did not raise ValueError")    # tests/test_dropin.py assumes it
+    return {"layers_imports": sorted(imports), "nets": nets}
+
+
 def main():
     lay = {}
     for c in LAYER_CASES:
         layer_case(*c, lay)
-    np.savez_compressed(os.path.join(HERE, "layers.npz"), **lay)
+    for part in sorted({k.split("/")[0].rsplit("_", 1)[0] for k in lay}):       # conv_bbb, conv_lrt, lin_bbb, lin_lrt
+        np.savez_compressed(os.path.join(HERE, f"layers_{part}.npz"),
+                            **{k: v for k, v in lay.items() if k.split("/")[0].rsplit("_", 1)[0] == part})
     mod = {}
     for c in MODEL_CASES:
         model_case(*c, mod)
     np.savez_compressed(os.path.join(HERE, "models.npz"), **mod)
-    print("layers.npz", os.path.getsize(os.path.join(HERE, "layers.npz")),
-          "models.npz", os.path.getsize(os.path.join(HERE, "models.npz")))
+    drop = {}
+    model_case("lenet_bbb_relu", BBBLeNet, "lenet", 3, 10, "bbb", "relu", 5, drop)
+    np.savez_compressed(os.path.join(HERE, "dropin.npz"), **drop)
+    with open(os.path.join(HERE, "dropin.json"), "w") as f:
+        json.dump(dropin_structure(), f, indent=1)
+        f.write("\n")
+    for f in sorted(glob.glob(os.path.join(HERE, "*.npz")) + glob.glob(os.path.join(HERE, "*.json"))):
+        print(os.path.basename(f), os.path.getsize(f))
     print("torch", torch.__version__)
 
 

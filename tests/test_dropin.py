@@ -1,61 +1,79 @@
-"""The reference's UNMODIFIED model files on top of this repo's `layers` package.
-Runs only where /root/reference exists (the build container); the GPU box uses models.py."""
-import importlib
+"""The reference's UNMODIFIED model files (models/BayesianModels/*.py) as consumers of this repo's `layers` package,
+checked against what tests/golden/make_golden.py recorded from the reference itself (tests/golden/dropin.*): the names
+the files import from `layers`, the child list they build (as `layers` exports / torch.nn types), the state_dict keys
+and shapes (so their checkpoints load here), and one of their forwards, run here on the engine."""
+import json
 import os
-import sys
 
+import numpy as np
 import pytest
 import torch
 
-from tests.conftest import ROOT
-from tests.util import CFG_PRIORS
+from tests.conftest import GOLDEN
+from tests.util import CFG_PRIORS, load_case, load_params_into, scale_err
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models")), reason="reference tree not present")
-
-
-@pytest.fixture()
-def ref_models():
-    """Import models.BayesianModels.* from the reference with OUR `layers` resolving first."""
-    saved_path, saved_mods = list(sys.path), dict(sys.modules)
-    for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
-        del sys.modules[k]
-    sys.path[:] = [ROOT] + [p for p in sys.path if p not in (ROOT, REF)] + [REF]
-    sys.dont_write_bytecode = True
-    try:
-        import layers
-        assert os.path.dirname(os.path.abspath(layers.__file__)) == os.path.join(ROOT, "layers")
-        mods = {n: importlib.import_module(f"models.BayesianModels.{m}") for n, m in
-                (("alexnet", "BayesianAlexNet"), ("lenet", "BayesianLeNet"), ("3conv3fc", "Bayesian3Conv3FC"))}
-        assert all(m.__file__.startswith(REF) for m in mods.values())
-        yield mods
-    finally:
-        sys.path[:] = saved_path
-        for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
-            del sys.modules[k]
+with open(os.path.join(GOLDEN, "dropin.json")) as f:
+    DROPIN = json.load(f)
 
 
-def test_reference_model_files_build_on_our_layers(ref_models):
+def _child(name, m):
+    import layers
+    for export in DROPIN["layers_imports"]:
+        if type(m) is getattr(layers, export):
+            return f"{name} layers.{export}"
+    return f"{name} nn.{type(m).__name__}"
+
+
+def test_reference_model_files_build_on_our_layers():
+    import layers
     import pytorch_bayesiancnn_b200 as bbb
     from pytorch_bayesiancnn_b200 import models as ours
-    pairs = [(ref_models["alexnet"].BBBAlexNet, ours.BBBAlexNet, 3), (ref_models["lenet"].BBBLeNet, ours.BBBLeNet, 3),
-             (ref_models["3conv3fc"].BBB3Conv3FC, ours.BBB3Conv3FC, 1)]
-    for ref_cls, our_cls, cin in pairs:
-        for lt in ("lrt", "bbb"):
-            net = ref_cls(10, cin, CFG_PRIORS, lt, "softplus")          # reference constructor, our layers
-            mine = our_cls(10, cin, CFG_PRIORS, lt, "softplus")
-            assert isinstance(net, bbb.ModuleWrapper)
-            assert list(net.state_dict().keys()) == list(mine.state_dict().keys())
-            assert [type(m).__name__ for m in net.children()] == [type(m).__name__ for m in mine.children()]
-            mine.load_state_dict(net.state_dict())                       # checkpoints are interchangeable
+    assert all(hasattr(layers, n) for n in DROPIN["layers_imports"])
+    assert len(DROPIN["nets"]) == 6
+    for case, rec in DROPIN["nets"].items():
+        cls = getattr(ours, rec["class"])
+        net = cls(10, rec["inputs"], CFG_PRIORS, rec["variant"], "softplus")
+        assert isinstance(net, bbb.ModuleWrapper)
+        assert [_child(n, m) for n, m in net.named_children()] == rec["children"], case
+        sd = net.state_dict()
+        assert [f"{k} {'x'.join(map(str, v.shape))}" for k, v in sd.items()] == rec["state_dict"], case
+        ckpt = {}                                                   # a checkpoint of the reference's layout loads strictly
+        for line in rec["state_dict"]:
+            k, shape = line.split(" ")
+            ckpt[k] = torch.randn([int(d) for d in shape.split("x")])
+        net.load_state_dict(ckpt)
+        assert all(torch.equal(net.state_dict()[k].cpu(), v) for k, v in ckpt.items()), case
         with pytest.raises(ValueError):
-            ref_cls(10, cin, CFG_PRIORS, "nope")
+            cls(10, rec["inputs"], CFG_PRIORS, "nope")
+        with pytest.raises(ValueError):
+            cls(10, rec["inputs"], CFG_PRIORS, rec["variant"], "nope")
 
 
 @pytest.mark.gpu
-def test_reference_model_files_run_on_the_engine(ref_models):
+def test_reference_model_files_run_on_the_engine():
+    """BBBLeNet with bbb layers and relu, recorded by the reference on its CPU layers, against the same net on the engine
+    with the reference's parameters and eps: the fp32 kernels at the whole-model bar; the default math with in-kernel
+    noise runs and is finite."""
+    import __graft_entry__ as g
+    g.build()
     import pytorch_bayesiancnn_b200 as bbb
-    net = ref_models["lenet"].BBBLeNet(10, 3, CFG_PRIORS, "bbb", "relu").cuda().train()
+    from pytorch_bayesiancnn_b200.models import BBBLeNet
+    from oracle import bbb_oracle as O
+    dev = torch.device("cuda:0")
+    with np.load(os.path.join(GOLDEN, "dropin.npz")) as z:
+        c = load_case(z, "lenet_bbb_relu")
+    key, inputs, outputs, variant, act, batch = [str(v) for v in c["meta"]]
+    inputs, outputs, batch = int(inputs), int(outputs), int(batch)
+    params = O.init_params(key, outputs, inputs, CFG_PRIORS, seed=123)
+    sums = [float(p[k].double().sum()) for p in params for k in ("W_mu", "W_rho", "bias_mu", "bias_rho")]
+    np.testing.assert_allclose(sums, c["param_sums"], rtol=0, atol=0)
+    net = load_params_into(BBBLeNet(outputs, inputs, CFG_PRIORS, variant, act), params).to(dev).train()
+    eps = O.draw_eps_like_reference(O.eps_shapes(key, outputs, inputs, variant, batch), seed=7)
+    with torch.no_grad(), bbb.external_eps(eps):
+        logits, kl = net(c["x"].to(dev))
+    assert scale_err(logits, c["logits"]) < 1e-4
+    assert abs(float(kl) - float(c["kl"])) <= 1e-5 * abs(float(c["kl"]))
+    net.set_flag("math", "auto")
     with torch.no_grad():
-        out, kl = net(torch.randn(5, 3, 32, 32, device="cuda"))
-    assert out.shape == (5, 10) and kl.dim() == 0 and torch.isfinite(out).all()
+        out, kl = net(torch.randn(batch, inputs, 32, 32, device=dev))
+    assert out.shape == (batch, outputs) and kl.dim() == 0 and torch.isfinite(out).all()

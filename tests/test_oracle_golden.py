@@ -11,11 +11,11 @@ CFG_PRIORS = {"prior_mu": 0, "prior_sigma": 0.1,
 
 
 def layer_names(g):
-    return sorted({k.split("/")[0] for k in g.files})
+    return sorted({k.split("/")[0] for k in g})
 
 
 def load_case(g, name):
-    d = {k.split("/", 1)[1]: g[k] for k in g.files if k.startswith(name + "/")}
+    d = {k.split("/", 1)[1]: g[k] for k in g if k.startswith(name + "/")}
     t = {k: (torch.from_numpy(v) if isinstance(v, np.ndarray) and v.dtype == np.float32 and v.ndim > 0 else v)
          for k, v in d.items()}
     return t
