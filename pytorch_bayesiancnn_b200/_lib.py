@@ -20,6 +20,7 @@ KL_REFERENCE, KL_TEXTBOOK = 0, 1
 ACT_NONE, ACT_SOFTPLUS, ACT_RELU = 0, 1, 2
 LAYOUT_NCHW_F32, LAYOUT_PACKED_BF16, LAYOUT_ROWMAJOR_F32 = 0, 1, 2
 FUSED_PREP_ONLY, FUSED_SKIP_PREP = 1, 2
+E_UNSUPPORTED = -2              # BBB_E_UNSUPPORTED: a valid call whose shape / mode this path does not take
 
 MATH_BY_NAME = {"fp32": MATH_FP32, "bf16": MATH_BF16_TC, "auto": MATH_AUTO, "tf32": MATH_TF32_TC}
 KL_BY_NAME = {"reference": KL_REFERENCE, "textbook": KL_TEXTBOOK}
@@ -46,7 +47,11 @@ class LayerDesc(C.Structure):
 
 
 class EngineError(RuntimeError):
-    pass
+    """``code``: the BBB_E_* status of the failed engine call (None for errors raised on the host side)."""
+
+    def __init__(self, msg, code=None):
+        super().__init__(msg)
+        self.code = code
 
 
 _lib = None
@@ -126,7 +131,7 @@ def lib():
 def check(rc: int, what: str):
     if rc != 0:
         msg = lib().bbb_last_error().decode("utf-8", "replace")
-        raise EngineError(f"{what} failed (code {rc}): {msg}")
+        raise EngineError(f"{what} failed (code {rc}): {msg}", rc)
 
 
 def launch_count() -> int:

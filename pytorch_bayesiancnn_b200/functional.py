@@ -174,6 +174,20 @@ def external_eps_active() -> bool:
     return _noise.queue is not None
 
 
+def draw_noise(variant, w_shape, b_shape, y_shape, device):
+    """(eps_a, eps_b, seed, stream_id, base) of one stochastic layer call.  Under ``external_eps`` it pops the
+    reference's draws (BBB: the weight eps, then the bias eps if ``b_shape`` is not None; LRT: one eps of the output
+    shape ``y_shape``); otherwise it takes the next Philox stream id (relative to the ``stream_base`` scalar, if any)."""
+    if not external_eps_active():
+        seed, stream_id = next_stream()
+        return None, None, seed, stream_id, _noise.base
+    if variant == L.VARIANT_LRT:
+        return _pop_eps(y_shape, device), None, 0, 0, None
+    eps_a = _pop_eps(w_shape, device)
+    eps_b = _pop_eps(b_shape, device) if b_shape is not None else None
+    return eps_a, eps_b, 0, 0, None
+
+
 # --------------------------------------------------------------------------- #
 # helpers
 # --------------------------------------------------------------------------- #
@@ -237,7 +251,10 @@ def workspace(device, desc=None, owner=None) -> torch.Tensor:
 
 def make_desc(x_shape, w_shape, conv, variant, sample, has_bias, prior_mu, prior_sigma,
               math=L.MATH_FP32, kl_convention=L.KL_REFERENCE, act=L.ACT_NONE,
-              act_dtype=L.DTYPE_F32) -> L.LayerDesc:
+              act_dtype=L.DTYPE_F32, pool=False, phase=0, fold=None) -> L.LayerDesc:
+    """The bbb_layer_desc of one layer call.  ``pool``: fused 2x2 max-pool epilogue; ``phase``: 0, FUSED_PREP_ONLY or
+    FUSED_SKIP_PREP; ``fold`` = (rows per MC sample, Philox stream stride) when MC samples are folded into the batch
+    (include/bbb_b200.h)."""
     d = L.LayerDesc()
     if conv is None:
         d.batch, d.in_channels, d.in_h, d.in_w = x_shape[0], x_shape[1], 1, 1
@@ -251,7 +268,13 @@ def make_desc(x_shape, w_shape, conv, variant, sample, has_bias, prior_mu, prior
         d.stride_h, d.stride_w, d.pad_h, d.pad_w, d.dil_h, d.dil_w = sh, sw, ph, pw, dh, dw
     d.variant, d.sample, d.has_bias = variant, int(bool(sample)), int(bool(has_bias))
     d.act_dtype, d.math, d.kl_convention, d.epilogue_act = act_dtype, math, kl_convention, act
-    d.pool_k = d.pool_s = 0
+    d.pool_k = d.pool_s = 2 if pool else 0
+    d.reserved[0] = phase
+    if fold is not None:
+        rows, stride = fold
+        d.reserved[1] = int(rows)
+        d.reserved[2] = C.c_int32(stride & 0xFFFFFFFF).value
+        d.reserved[3] = C.c_int32((stride >> 32) & 0xFFFFFFFF).value
     d.prior_mu, d.prior_sigma = float(prior_mu), float(prior_sigma)
     return d
 
@@ -267,15 +290,13 @@ def out_hw(h, w, kh, kw, conv):
 _TC_K_MAX = 8192          # the gather kernel keeps an 8-byte table entry per reduction index in shared memory
 
 
-_tc_math = L.MATH_BF16_TC          # operand type of the backward contractions (set per call by _backward_tc)
-
-
-def _tc_contract(x, w, conv):
+def _tc_contract(x, w, conv, math):
     """Plain (mean-only, bias-free) conv2d / linear of fp32 `x` with the fp32 tensor `w` on the tcgen05 layer kernel
-    (bf16 or tf32 operands like the layer's forward, fp32 TMEM accumulators): the engine's forward with sample=0, no KL."""
+    (`math`: bf16 or tf32 operands like the layer's forward, fp32 TMEM accumulators): the engine's forward with
+    sample=0, no KL."""
     lib = L.lib()
     x, w = x.contiguous(), w.contiguous()
-    d = make_desc(tuple(x.shape), tuple(w.shape), conv, L.VARIANT_BBB, False, False, 0.0, 1.0, _tc_math)
+    d = make_desc(tuple(x.shape), tuple(w.shape), conv, L.VARIANT_BBB, False, False, 0.0, 1.0, math)
     if conv is None:
         y = torch.empty(x.shape[0], w.shape[0], dtype=torch.float32, device=x.device)
         fn = lib.bbb_linear_forward
@@ -290,11 +311,11 @@ def _tc_contract(x, w, conv):
     return y
 
 
-def _tc_dgrad(g, w, conv, x_shape):
+def _tc_dgrad(g, w, conv, x_shape, math):
     """d x of y = conv(x, w): the full correlation of (zero-inserted) g with the flipped, channel-transposed kernel --
     itself a stride-1 convolution, so it runs on the same tcgen05 layer kernel."""
     if conv is None:
-        return _tc_contract(g, w.t(), None)                               # [B,N] x [K,N]^T -> [B,K]
+        return _tc_contract(g, w.t(), None, math)                         # [B,N] x [K,N]^T -> [B,K]
     (sh, sw), (ph, pw), (dh, dw) = conv
     kh, kw = w.shape[2], w.shape[3]
     H, W = x_shape[2], x_shape[3]
@@ -309,15 +330,15 @@ def _tc_dgrad(g, w, conv, x_shape):
         gu[:, :, 0:(OH - 1) * sh + 1:sh, 0:(OW - 1) * sw + 1:sw] = g
         g = gu
     wt = w.flip(2, 3).transpose(0, 1)
-    return _tc_contract(g, wt, ((1, 1), (qh, qw), (dh, dw)))
+    return _tc_contract(g, wt, ((1, 1), (qh, qw), (dh, dw)), math)
 
 
-def _tc_wgrad(x, g, conv, w_shape):
+def _tc_wgrad(x, g, conv, w_shape, math):
     """d w of y = conv(x, w): a convolution with the batch as the reduction ("channel") axis -- input x^T [C,B,H,W],
     kernel g^T [N,B,OH,OW], stride <-> dilation swapped -- on the tcgen05 layer kernel.  Deterministic (no atomics);
     the batch is cut so that the reduction index fits the kernel's shared-memory table and the partial results summed."""
     if conv is None:
-        out = _tc_contract(x.t(), g.t(), None)                             # [K,B] x [N,B]^T -> [K,N]
+        out = _tc_contract(x.t(), g.t(), None, math)                       # [K,B] x [N,B]^T -> [K,N]
         return out.t()
     (sh, sw), (ph, pw), (dh, dw) = conv
     kh, kw = w_shape[2], w_shape[3]
@@ -327,13 +348,13 @@ def _tc_wgrad(x, g, conv, w_shape):
     for b0 in range(0, B, per):
         xt = x[b0:b0 + per].transpose(0, 1)
         gt = g[b0:b0 + per].transpose(0, 1)
-        part = _tc_contract(xt, gt, ((dh, dw), (ph, pw), (sh, sw)))[:, :, :kh, :kw]
+        part = _tc_contract(xt, gt, ((dh, dw), (ph, pw), (sh, sw)), math)[:, :, :kh, :kw]
         acc = part if acc is None else acc + part
     return acc.transpose(0, 1)
 
 
 def _tc_backward_ok(cfg):
-    return cfg["math"] in (L.MATH_BF16_TC, L.MATH_AUTO, L.MATH_TF32_TC) and os.environ.get("BBB_B200_BWD", "tc") != "simt"
+    return cfg["math"] in (L.MATH_BF16_TC, L.MATH_AUTO, L.MATH_TF32_TC)
 
 
 # --------------------------------------------------------------------------- #
@@ -369,20 +390,9 @@ class BayesLayerFn(torch.autograd.Function):
             yshape = (x.shape[0], W_mu.shape[0], oh, ow)
         y = torch.empty(yshape, dtype=torch.float32, device=dev)
         kl = torch.empty((), dtype=torch.float32, device=dev)
-        eps_a = eps_b = None
-        seed = stream_id = 0
-        base = None
-        if sample:
-            if external_eps_active():
-                if variant == L.VARIANT_BBB:
-                    eps_a = _pop_eps(W_mu.shape, dev)
-                    if has_bias:
-                        eps_b = _pop_eps(bias_mu.shape, dev)
-                else:
-                    eps_a = _pop_eps(yshape, dev)
-            else:
-                seed, stream_id = next_stream()
-                base = _noise.base
+        eps_a, eps_b, seed, stream_id, base = (
+            draw_noise(variant, W_mu.shape, bias_mu.shape if has_bias else None, yshape, dev) if sample
+            else (None, None, 0, 0, None))
         need_grad = any(ctx.needs_input_grad[:5])      # grad mode is off inside Function.forward
         act_std = None
         if variant == L.VARIANT_LRT and sample and need_grad:
@@ -418,7 +428,7 @@ class BayesLayerFn(torch.autograd.Function):
             try:
                 out = BayesLayerFn._backward_tc(ctx, gy.contiguous().float())
             except L.EngineError as e:
-                if "code -2" not in str(e):                # BBB_E_UNSUPPORTED: a shape the tcgen05 kernel does not take
+                if e.code != L.E_UNSUPPORTED:              # a shape the tcgen05 kernel does not take
                     raise
                 out = None
             if out is not None:
@@ -467,8 +477,7 @@ class BayesLayerFn(torch.autograd.Function):
         cfg = ctx.cfg
         conv, variant, sample = cfg["conv"], cfg["variant"], cfg["sample"]
         dev = x.device
-        global _tc_math
-        _tc_math = L.MATH_TF32_TC if cfg["math"] == L.MATH_TF32_TC else L.MATH_BF16_TC     # same operand type as the forward
+        math = L.MATH_TF32_TC if cfg["math"] == L.MATH_TF32_TC else L.MATH_BF16_TC      # same operand type as the forward
         seed, stream_id, base = ctx.noise
         if base is not None:
             stream_id = int(stream_id) + int(base.item())
@@ -478,7 +487,7 @@ class BayesLayerFn(torch.autograd.Function):
         gb_mu = gb_rho = None
         red = (0,) if conv is None else (0, 2, 3)
         if variant == L.VARIANT_LRT:
-            gw_mu = _tc_wgrad(x, gy, conv, W_mu.shape)
+            gw_mu = _tc_wgrad(x, gy, conv, W_mu.shape, math)
             if sample:
                 if eps_a is None:
                     z = philox_normal(gy.numel(), seed, stream_id, 0, device=dev)
@@ -486,16 +495,16 @@ class BayesLayerFn(torch.autograd.Function):
                 else:
                     eps = eps_a
                 gv = gy * eps / (2.0 * act_std)
-                gw_rho = _tc_wgrad(x * x, gv, conv, W_mu.shape) * (2.0 * sig * dsig)
+                gw_rho = _tc_wgrad(x * x, gv, conv, W_mu.shape, math) * (2.0 * sig * dsig)
             else:
                 gv, gw_rho = None, torch.zeros_like(W_rho)
             gx = None
             if need_x:
-                gx = _tc_dgrad(gy, W_mu, conv, x.shape)
+                gx = _tc_dgrad(gy, W_mu, conv, x.shape, math)
                 if gx is None:
                     return None
                 if sample:
-                    gx2 = _tc_dgrad(gv, sig * sig, conv, x.shape)
+                    gx2 = _tc_dgrad(gv, sig * sig, conv, x.shape, math)
                     gx = gx + 2.0 * x * gx2
             if ctx.has_bias:
                 gb_mu = gy.sum(red)
@@ -511,11 +520,11 @@ class BayesLayerFn(torch.autograd.Function):
                 W = W_mu + ew * sig
             else:
                 ew, W = None, W_mu
-            gw_mu = _tc_wgrad(x, gy, conv, W_mu.shape)
+            gw_mu = _tc_wgrad(x, gy, conv, W_mu.shape, math)
             gw_rho = gw_mu.reshape(W_mu.shape) * ew * dsig if sample else torch.zeros_like(W_rho)
             gx = None
             if need_x:
-                gx = _tc_dgrad(gy, W, conv, x.shape)
+                gx = _tc_dgrad(gy, W, conv, x.shape, math)
                 if gx is None:
                     return None
             if ctx.has_bias:

@@ -14,7 +14,6 @@ child-by-child path.
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import torch
 from torch import nn
@@ -26,6 +25,20 @@ from . import functional as Fn
 class _Step:
     __slots__ = ("layer", "act", "pool", "conv", "in_shape", "in_layout", "prev_hw", "out_layout", "out_chw",
                  "eps_shape", "linear", "batch")
+
+    def desc(self, phase=0, fold=None):
+        """The layer call's descriptor (ModuleWrapper calls its children with sample=True: SURVEY D6)."""
+        m = self.layer
+        return Fn.make_desc((self.batch,) + self.in_shape, tuple(m.W_mu.shape), self.conv, m._variant, True,
+                            m.use_bias, m.prior_mu, m.prior_sigma, L.MATH_BF16_TC, L.KL_BY_NAME[m.kl_convention],
+                            self.act, pool=self.pool, phase=phase, fold=fold)
+
+    def noise(self):
+        """The layer call's noise, drawn exactly as the per-layer path draws it."""
+        m, (cout, oh, ow) = self.layer, self.eps_shape
+        y_shape = (self.batch, cout) if self.linear else (self.batch, cout, oh, ow)
+        return Fn.draw_noise(m._variant, m.W_mu.shape, m.bias_mu.shape if m.use_bias else None, y_shape,
+                             m.W_mu.device)
 
 
 def _act_code(m):
@@ -72,11 +85,9 @@ def plan(children, x_shape, fold=None):
         else:
             if m.in_channels != c:
                 return None
-            (sh, sw), (ph, pw), (dh, dw) = st.conv
-            if (dh, dw) != (1, 1):
+            if st.conv[2] != (1, 1):            # dilation
                 return None
-            kh, kw = m.kernel_size
-            oh, ow = (h + 2 * ph - kh) // sh + 1, (w + 2 * pw - kw) // sw + 1
+            oh, ow = Fn.out_hw(h, w, *m.kernel_size, st.conv)
             if oh < 1 or ow < 1:
                 return None
             if lay == "packed" and (h * w > 64 or c % 64):
@@ -117,9 +128,9 @@ def plan(children, x_shape, fold=None):
     # discover an unsupported shape after noise was drawn and prep kernels were enqueued on side streams
     lib = L.lib()
     for st in steps:
-        d = _step_desc(st, 0, fold)
+        d = st.desc(fold=fold)
         rc = lib.bbb_fused_supported(C.byref(d), st.in_layout, _in_pitch(st), st.prev_hw, st.out_layout, _out_pitch(st))
-        if rc == -2:                            # BBB_E_UNSUPPORTED: not fusable, the caller runs child by child
+        if rc == L.E_UNSUPPORTED:               # not fusable, the caller runs child by child
             return None
         L.check(rc, "bbb_fused_supported")
     return steps
@@ -135,36 +146,8 @@ def _out_pitch(st):
     return cout * oh * ow if st.out_layout == L.LAYOUT_PACKED_BF16 else 0
 
 
-def _step_desc(st, phase, fold=None):
-    m = st.layer
-    cin, h, w = st.in_shape
-    d = L.LayerDesc()
-    d.batch, d.in_channels, d.in_h, d.in_w = st.batch, cin, h, w
-    if st.linear:
-        d.out_channels, d.kernel_h, d.kernel_w = m.out_features, 1, 1
-        d.stride_h = d.stride_w = d.dil_h = d.dil_w = 1
-        d.pad_h = d.pad_w = 0
-    else:
-        (sh, sw), (ph, pw), (dh, dw) = st.conv
-        d.out_channels, d.kernel_h, d.kernel_w = m.out_channels, m.kernel_size[0], m.kernel_size[1]
-        d.stride_h, d.stride_w, d.pad_h, d.pad_w, d.dil_h, d.dil_w = sh, sw, ph, pw, dh, dw
-    d.variant, d.sample, d.has_bias = m._variant, 1, int(m.use_bias)     # ModuleWrapper calls children with sample=True (SURVEY D6)
-    d.act_dtype, d.math = L.DTYPE_F32, L.MATH_BF16_TC
-    d.kl_convention = L.KL_BY_NAME[m.kl_convention]
-    d.epilogue_act = st.act
-    d.pool_k = d.pool_s = 2 if st.pool else 0
-    d.reserved[0] = phase
-    if fold is not None:                    # MC samples folded into the batch (include/bbb_b200.h)
-        rows, stride = fold
-        d.reserved[1] = int(rows)
-        d.reserved[2] = C.c_int32(stride & 0xFFFFFFFF).value
-        d.reserved[3] = C.c_int32((stride >> 32) & 0xFFFFFFFF).value
-    d.prior_mu, d.prior_sigma = float(m.prior_mu), float(m.prior_sigma)
-    return d
-
-
 _side_streams: dict = {}
-_direct = {"out": None, "terms": False}
+_direct: dict = {}                  # run()'s keyword arguments inside a direct_output block
 
 
 class direct_output:
@@ -180,7 +163,7 @@ class direct_output:
 
     def __enter__(self):
         self.prev = dict(_direct)
-        _direct.update(out=self.out, terms=True, owner=self, kl_buf=self.kl_buf)
+        _direct.update(out=self.out, terms=True, owner=self, kls_out=self.kl_buf)
         return self
 
     def __exit__(self, *exc):
@@ -196,22 +179,19 @@ def _side_stream(dev, i=0):
     return st
 
 
-def _prep_chains():
-    return max(1, int(os.environ.get("BBB_B200_PREP_CHAINS", "3")))
+_PREP_CHAINS = 3        # serial side streams the parameter preps are dealt over (see run)
 
 
-def run(steps, x: torch.Tensor, overlap_prep: bool = True):
-    return _run(steps, x, overlap_prep, _direct.get("out"), _direct.get("terms", False), _direct.get("owner"),
-                kls_out=_direct.get("kl_buf"))
-
-
-def _run(steps, x, overlap_prep, out, terms, owner, fold=None, kls_out=None):
-    """Execute a planned chain.  Returns (network output fp32, summed KL 0-dim tensor).
+def run(steps, x: torch.Tensor, *, out=None, terms=False, owner=None, fold=None, kls_out=None):
+    """Execute a planned chain.  Returns (network output fp32, summed KL 0-dim tensor); with ``terms`` the per-layer
+    KL scalars un-summed instead of their sum, and ``owner.used`` is set.  ``out``: a [B, C] fp32 buffer the last
+    layer writes its output into when it can; ``fold``: as in plan(); ``kls_out``: a vector the per-layer KL scalars
+    are written to.  ``ModuleWrapper`` passes the keywords of the enclosing ``direct_output`` block.
 
     The parameter-only half of every layer (softplus / eps / bf16 operand tiles / KL) runs on side
     streams (parallel branches of a captured graph), joined to the GEMM chain by events, so only the
     first layer's prep is on the activation critical path.  The preps are issued in layer order over
-    a few serial chains (default 3: layers 1,4 / 2,5 / 3) rather than all at once: six concurrent prep
+    a few serial chains (3: layers 1,4 / 2,5 / 3) rather than all at once: six concurrent prep
     grids fill the machine and the first layer's prep -- the one the GEMM chain is waiting for -- was
     scheduled last (measured with tools/timeline.py: first GEMM at 24 us instead of ~20).  The KL sum
     depends on the preps only and runs on the side as well."""
@@ -219,42 +199,35 @@ def _run(steps, x, overlap_prep, out, terms, owner, fold=None, kls_out=None):
     kls = kls_out[:len(steps)] if kls_out is not None else torch.empty(len(steps), dtype=torch.float32, device=dev)
     snap = Fn.noise_snapshot()
     main = torch.cuda.current_stream(dev)
-    chains = [_side_stream(dev, c) for c in range(min(_prep_chains(), len(steps)))] if overlap_prep else []
+    chains = [_side_stream(dev, c) for c in range(min(_PREP_CHAINS, len(steps)))]
     forked = False
     try:
         if fold is not None and Fn.external_eps_active():
             raise L.EngineError("MC-sample folding draws its noise in-kernel (no external eps)")
-        noise = [_draw_noise(st, x.shape[0], dev) for st in steps]
-        if overlap_prep:
-            for side in chains:
-                side.wait_stream(main)
-            forked = True
-            # The FIRST layer's prep stays on the main stream, right in front of its GEMM kernel: launched with programmatic
-            # serialization the GEMM kernel's CTAs start while the prep runs and stage their input images meanwhile
-            # (conv_s4_tc.cuh); only its weight producer waits for the prep.  The other preps go to the side chains.
-            events = [None] * len(steps)
-            first_on_main = os.environ.get("BBB_B200_PREP0_MAIN", "1") == "1"
-            ev0 = None
-            if first_on_main:
-                run_step(steps[0], None, None, None, 0, kl=kls[0], noise=noise[0], phase=L.FUSED_PREP_ONLY, fold=fold)
-                ev0 = torch.cuda.Event()
-                ev0.record(main)
-            for i, st in enumerate(steps):
-                if i == 0 and first_on_main:
-                    continue
-                side = chains[(i - 1) % len(chains)] if first_on_main else chains[i % len(chains)]
-                with torch.cuda.stream(side):
-                    run_step(st, None, None, None, 0, kl=kls[i], noise=noise[i], phase=L.FUSED_PREP_ONLY, fold=fold)
-                    ev = torch.cuda.Event()
-                    ev.record(side)
-                    events[i] = ev
-            for side in chains[1:]:
-                chains[0].wait_stream(side)
-            if not terms:
-                with torch.cuda.stream(chains[0]):
-                    if ev0 is not None:
-                        chains[0].wait_event(ev0)
-                    kl_total = kls.sum()
+        noise = [st.noise() for st in steps]
+        for side in chains:
+            side.wait_stream(main)
+        forked = True
+        # The FIRST layer's prep stays on the main stream, right in front of its GEMM kernel: launched with programmatic
+        # serialization the GEMM kernel's CTAs start while the prep runs and stage their input images meanwhile
+        # (conv_s4_tc.cuh); only its weight producer waits for the prep.  The other preps go to the side chains.
+        events = [None] * len(steps)
+        run_step(steps[0], None, None, None, 0, kl=kls[0], noise=noise[0], phase=L.FUSED_PREP_ONLY, fold=fold)
+        ev0 = torch.cuda.Event()
+        ev0.record(main)
+        for i in range(1, len(steps)):
+            side = chains[(i - 1) % len(chains)]
+            with torch.cuda.stream(side):
+                run_step(steps[i], None, None, None, 0, kl=kls[i], noise=noise[i], phase=L.FUSED_PREP_ONLY, fold=fold)
+                ev = torch.cuda.Event()
+                ev.record(side)
+                events[i] = ev
+        for side in chains[1:]:
+            chains[0].wait_stream(side)
+        if not terms:
+            with torch.cuda.stream(chains[0]):
+                chains[0].wait_event(ev0)
+                kl_total = kls.sum()
         cur, cur_sq, cur_pitch = x.contiguous().float(), None, 0
         last = steps[-1]
         take = (out is not None and last.out_layout == L.LAYOUT_ROWMAJOR_F32 and out.is_contiguous()
@@ -262,19 +235,14 @@ def _run(steps, x, overlap_prep, out, terms, owner, fold=None, kls_out=None):
         for i, st in enumerate(steps):
             nxt = steps[i + 1].layer if i + 1 < len(steps) else None
             y_into = out if (take and i == len(steps) - 1) else None
-            if overlap_prep:
-                if events[i] is not None:
-                    main.wait_event(events[i])
-                cur, cur_sq, cur_pitch = run_step(st, nxt, cur, cur_sq, cur_pitch, kl=kls[i], noise=noise[i],
-                                                  phase=L.FUSED_SKIP_PREP, y_into=y_into, fold=fold)
-            else:
-                cur, cur_sq, cur_pitch = run_step(st, nxt, cur, cur_sq, cur_pitch, kl=kls[i], noise=noise[i], y_into=y_into, fold=fold)
+            if events[i] is not None:
+                main.wait_event(events[i])
+            cur, cur_sq, cur_pitch = run_step(st, nxt, cur, cur_sq, cur_pitch, kl=kls[i], noise=noise[i],
+                                              phase=L.FUSED_SKIP_PREP, y_into=y_into, fold=fold)
         if terms:
             kl_total = kls
             if owner is not None:
                 owner.used = True
-        elif not overlap_prep:
-            kl_total = kls.sum()
     except BaseException:
         Fn.noise_restore(snap)                 # a retry / fallback sees the stream ids and eps queue it would have seen
         raise
@@ -286,26 +254,6 @@ def _run(steps, x, overlap_prep, out, terms, owner, fold=None, kls_out=None):
     return cur, kl_total
 
 
-def _draw_noise(st, B, dev):
-    """(eps_a, eps_b, seed, stream_id, base) for one layer call, consuming the external-eps
-    queue / the Philox stream counter exactly like the unfused layer would."""
-    m = st.layer
-    eps_a = eps_b = None
-    seed = stream_id = 0
-    base = None
-    if Fn.external_eps_active():
-        if m._variant == L.VARIANT_LRT:
-            eps_a = Fn._pop_eps((B,) + st.eps_shape if not st.linear else (B, st.eps_shape[0]), dev)
-        else:
-            eps_a = Fn._pop_eps(m.W_mu.shape, dev)
-            if m.use_bias:
-                eps_b = Fn._pop_eps(m.bias_mu.shape, dev)
-    else:
-        seed, stream_id = Fn.next_stream()
-        base = Fn._noise.base
-    return eps_a, eps_b, seed, stream_id, base
-
-
 def run_step(st, nxt, cur, cur_sq, cur_pitch, kl=None, noise=None, phase=0, y_into=None, fold=None):
     """One fused layer call: (y, y_sq, pitch) = step(cur, cur_sq).  phase: 0 = prep + GEMM,
     FUSED_PREP_ONLY / FUSED_SKIP_PREP = one half (see include/bbb_b200.h)."""
@@ -313,35 +261,34 @@ def run_step(st, nxt, cur, cur_sq, cur_pitch, kl=None, noise=None, phase=0, y_in
     m = st.layer
     dev = m.W_mu.device
     B = st.batch                                    # (packed inputs carry rows padded to the 128-row tile)
-    if True:
-        cin, h, w = st.in_shape
-        d = _step_desc(st, phase, fold)
-        in_pitch = cur_pitch if st.in_layout == L.LAYOUT_NCHW_F32 else cin * h * w
-        cout, oh, ow = st.out_chw
-        if phase == L.FUSED_PREP_ONLY:
-            pitch, y, y_sq = cout * oh * ow if st.out_layout == L.LAYOUT_PACKED_BF16 else 0, None, None
-        elif st.out_layout == L.LAYOUT_PACKED_BF16:
-            pitch = cout * oh * ow                   # tiled packed: [ceil(B/128)][F/64][planes][128 x 64] bf16
-            planes = 2 if (nxt is not None and nxt._variant == L.VARIANT_LRT) else 1
-            y = torch.empty((B + 127) // 128 * 128, pitch * planes, dtype=torch.bfloat16, device=dev)
-            y_sq = y.view(-1)[128 * 64:] if planes == 2 else None      # x^2 blocks interleaved behind the x blocks
-        elif st.out_layout == L.LAYOUT_ROWMAJOR_F32:
-            pitch, y, y_sq = 0, (y_into if y_into is not None else torch.empty(B, cout, dtype=torch.float32, device=dev)), None
-        else:
-            pitch, y, y_sq = 0, torch.empty(B, cout, oh, ow, dtype=torch.float32, device=dev), None
-        if kl is None:
-            kl = torch.empty((), dtype=torch.float32, device=dev)
-        if noise is None:
-            noise = _draw_noise(st, B, dev)
-        eps_a, eps_b, seed, stream_id, base = noise
-        ws = Fn.workspace(dev, d, m)
-        rc = lib.bbb_layer_forward_fused(
-            C.byref(d), Fn._ptr(cur), Fn._ptr(cur_sq), st.in_layout, in_pitch, st.prev_hw,
-            Fn._ptr(m.W_mu), Fn._ptr(m.W_rho), Fn._ptr(m.bias_mu), Fn._ptr(m.bias_rho),
-            Fn._ptr(y), Fn._ptr(y_sq), st.out_layout, pitch, Fn._ptr(kl), Fn._ptr(eps_a), Fn._ptr(eps_b),
-            C.c_uint64(seed), C.c_uint64(stream_id), Fn._ptr(base), Fn._ptr(ws), C.c_size_t(ws.numel()),
-            Fn._stream(dev))
-        L.check(rc, "bbb_layer_forward_fused")
-        if phase != L.FUSED_SKIP_PREP:
-            m._kl_cache = (kl, m._versions(), torch.is_grad_enabled())
-        return y, y_sq, pitch
+    cin, h, w = st.in_shape
+    d = st.desc(phase, fold)
+    in_pitch = cur_pitch if st.in_layout == L.LAYOUT_NCHW_F32 else cin * h * w
+    cout, oh, ow = st.out_chw
+    if phase == L.FUSED_PREP_ONLY:
+        pitch, y, y_sq = cout * oh * ow if st.out_layout == L.LAYOUT_PACKED_BF16 else 0, None, None
+    elif st.out_layout == L.LAYOUT_PACKED_BF16:
+        pitch = cout * oh * ow                   # tiled packed: [ceil(B/128)][F/64][planes][128 x 64] bf16
+        planes = 2 if (nxt is not None and nxt._variant == L.VARIANT_LRT) else 1
+        y = torch.empty((B + 127) // 128 * 128, pitch * planes, dtype=torch.bfloat16, device=dev)
+        y_sq = y.view(-1)[128 * 64:] if planes == 2 else None      # x^2 blocks interleaved behind the x blocks
+    elif st.out_layout == L.LAYOUT_ROWMAJOR_F32:
+        pitch, y, y_sq = 0, (y_into if y_into is not None else torch.empty(B, cout, dtype=torch.float32, device=dev)), None
+    else:
+        pitch, y, y_sq = 0, torch.empty(B, cout, oh, ow, dtype=torch.float32, device=dev), None
+    if kl is None:
+        kl = torch.empty((), dtype=torch.float32, device=dev)
+    if noise is None:
+        noise = st.noise()
+    eps_a, eps_b, seed, stream_id, base = noise
+    ws = Fn.workspace(dev, d, m)
+    rc = lib.bbb_layer_forward_fused(
+        C.byref(d), Fn._ptr(cur), Fn._ptr(cur_sq), st.in_layout, in_pitch, st.prev_hw,
+        Fn._ptr(m.W_mu), Fn._ptr(m.W_rho), Fn._ptr(m.bias_mu), Fn._ptr(m.bias_rho),
+        Fn._ptr(y), Fn._ptr(y_sq), st.out_layout, pitch, Fn._ptr(kl), Fn._ptr(eps_a), Fn._ptr(eps_b),
+        C.c_uint64(seed), C.c_uint64(stream_id), Fn._ptr(base), Fn._ptr(ws), C.c_size_t(ws.numel()),
+        Fn._stream(dev))
+    L.check(rc, "bbb_layer_forward_fused")
+    if phase != L.FUSED_SKIP_PREP:
+        m._kl_cache = (kl, m._versions(), torch.is_grad_enabled())
+    return y, y_sq, pitch

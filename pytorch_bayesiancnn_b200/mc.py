@@ -217,8 +217,8 @@ class MCForward:
             kl_ptr, n_kl = None, 0
             if self.fold_steps is not None:
                 with Fn.stream_base(base), Fn.mc_sample(self.ids[0], self.seed):
-                    _, kls = fused._run(self.fold_steps, x, True, logits_buf.view(len(self.ids) * self.B, self.C), True, None,
-                                        fold=self.fold, kls_out=kl_buf)
+                    _, kls = fused.run(self.fold_steps, x, out=logits_buf.view(len(self.ids) * self.B, self.C), terms=True,
+                                       fold=self.fold, kls_out=kl_buf)
                 self._kl_terms = kls
                 kl_ptr, n_kl = Fn._ptr(kls), kls.numel()
             for k, j in enumerate(self.ids if self.fold_steps is None else ()):
@@ -252,8 +252,6 @@ class MCForward:
         L.check(rc, "bbb_mc_exchange")
 
     def _capture(self, warmup: int = 2):
-        from .graph import _STRIDE
-        dev = self.dev
         # several steps in flight: the tap-GEMM layers take their 128-column tiles wherever Cout allows (throughput over the
         # latency of one step; the choice is made at launch = capture time, include/bbb_b200.h bbb_set_wide_tiles)
         prev_wide = L.lib().bbb_set_wide_tiles(1 if self.inflight > 1 else 0)

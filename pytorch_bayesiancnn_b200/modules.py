@@ -70,9 +70,9 @@ class ModuleWrapper(nn.Module):
         if steps is None:
             return None
         try:
-            return fused.run(steps, x)          # (output, summed KL)
+            return fused.run(steps, x, **fused._direct)     # (output, summed KL)
         except L.EngineError as e:
-            if "code -2" not in str(e):                    # anything but BBB_E_UNSUPPORTED is a real error
+            if e.code != L.E_UNSUPPORTED:                  # anything else is a real error
                 raise
             plans[key] = None
             return None

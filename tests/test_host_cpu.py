@@ -41,6 +41,7 @@ def test_header_enums_match_the_python_mirror_and_tile_policy_is_host_only(built
     assert (val("BBB_MATH_FP32"), val("BBB_MATH_BF16_TC"), val("BBB_MATH_AUTO"), val("BBB_MATH_TF32_TC")) == \
         (_lib.MATH_FP32, _lib.MATH_BF16_TC, _lib.MATH_AUTO, _lib.MATH_TF32_TC)
     assert (val("BBB_MC_MOMENTS"), val("BBB_MC_NORMALIZED")) == (_lib.MC_MOMENTS, _lib.MC_NORMALIZED)
+    assert val("BBB_E_UNSUPPORTED") == _lib.E_UNSUPPORTED
     assert set(_lib.MATH_BY_NAME) == {"fp32", "bf16", "tf32", "auto"}
     lib = _lib.lib()
     prev = lib.bbb_set_wide_tiles(1)
