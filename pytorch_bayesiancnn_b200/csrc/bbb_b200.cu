@@ -230,6 +230,15 @@ int bbb_fused_supported(const bbb_layer_desc* d, int32_t in_layout, int32_t in_p
     return fused_check(d, g, in_layout, in_pitch, prev_hw, out_layout, out_pitch);
 }
 
+/* which kernel runs a checked fused step: the stride-4 first-layer kernel, the gather kernel or the tap-GEMM */
+enum { FUSED_KERNEL_CONV_S4 = 0, FUSED_KERNEL_GATHER = 1, FUSED_KERNEL_TAP_GEMM = 2 };
+static int fused_kernel(const bbb_layer_desc* d, const bbb::Geom& g, int32_t in_layout, int32_t out_layout) {
+    if (in_layout == BBB_LAYOUT_PACKED_BF16) return FUSED_KERNEL_TAP_GEMM;
+    static const bool s4_on = [] { const char* e = getenv("BBB_B200_CONV1_DIRECT"); return !(e && e[0] == '0'); }();
+    if (s4_on && bbb::conv_s4_supported(*d, g, d->pool_k != 0, out_layout == BBB_LAYOUT_PACKED_BF16)) return FUSED_KERNEL_CONV_S4;
+    return FUSED_KERNEL_GATHER;
+}
+
 int bbb_layer_forward_fused(const bbb_layer_desc* d, const void* x, const void* x_sq, int32_t in_layout,
                             int32_t in_pitch, int32_t prev_hw, const float* W_mu, const float* W_rho,
                             const float* bias_mu, const float* bias_rho, void* y, void* y_sq, int32_t out_layout,
@@ -257,8 +266,8 @@ int bbb_layer_forward_fused(const bbb_layer_desc* d, const void* x, const void* 
     cudaStream_t st = (cudaStream_t)stream;
     const int out_mode = out_layout == BBB_LAYOUT_PACKED_BF16 ? 0 : (out_layout == BBB_LAYOUT_ROWMAJOR_F32 ? 1 : 2);
     int nl = 0;
-    static const bool s4_on = [] { const char* e = getenv("BBB_B200_CONV1_DIRECT"); return !(e && e[0] == '0'); }();
-    if (in_layout == BBB_LAYOUT_NCHW_F32 && s4_on && bbb::conv_s4_supported(*d, g, pool, out_mode == 0)) {
+    const int kernel = fused_kernel(d, g, in_layout, out_layout);
+    if (kernel == FUSED_KERNEL_CONV_S4) {
         // stride-4 first layer: the tensor core reads its A operand straight from the staged image (conv_s4_tc.cuh)
         bbb::S4Args a;
         a.g = g; a.x = (const float*)x; a.w_mu = W_mu; a.w_rho = W_rho; a.b_mu = bias_mu; a.b_rho = bias_rho;
@@ -274,7 +283,7 @@ int bbb_layer_forward_fused(const bbb_layer_desc* d, const void* x, const void* 
         a.tl_prep = tl_slot(!skip_prep, "conv_s4_prep", g); a.tl_gemm = tl_slot(!prep_only, "conv_s4", g);
         cudaError_t e = bbb::launch_conv_s4(a, st, !skip_prep, !prep_only, &nl);
         if (e != cudaSuccess) return cuda_fail(e, "conv_s4 launch");
-    } else if (in_layout == BBB_LAYOUT_NCHW_F32) {
+    } else if (kernel == FUSED_KERNEL_GATHER) {
         if (fold.rows) return fail(BBB_E_UNSUPPORTED, "MC-sample folding is not available on the gather path");
         bbb::TcArgs a;
         a.g = g; a.x = x; a.w_mu = W_mu; a.w_rho = W_rho; a.b_mu = bias_mu; a.b_rho = bias_rho;
@@ -291,7 +300,7 @@ int bbb_layer_forward_fused(const bbb_layer_desc* d, const void* x, const void* 
         a.tl_prep = tl_slot(!skip_prep, "weight_prep", g); a.tl_gemm = tl_slot(!prep_only, "gemm_tc", g);
         cudaError_t e = bbb::launch_fwd_tc(a, st, sm_count(), &nl);
         if (e != cudaSuccess) return cuda_fail(e, "fused gather launch");
-    } else if (in_layout == BBB_LAYOUT_PACKED_BF16) {
+    } else {
         bbb::FusedArgs a;
         a.g = g; a.variant = d->variant; a.sample = d->sample; a.has_bias = d->has_bias; a.act = d->epilogue_act;
         a.kl_convention = d->kl_convention; a.prior_mu = d->prior_mu; a.prior_sigma = d->prior_sigma;
@@ -307,8 +316,6 @@ int bbb_layer_forward_fused(const bbb_layer_desc* d, const void* x, const void* 
         const char* why = "";
         cudaError_t e = bbb::launch_fused(a, x, x_sq, st, &nl, &why, !skip_prep, !prep_only, sm_count(), g_wide_tiles.load() != 0);
         if (e != cudaSuccess) return fail(BBB_E_CUDA, "fused tap-GEMM launch: %s %s", cudaGetErrorString(e), why);
-    } else {
-        return fail(BBB_E_INVALID, "bad in_layout %d", in_layout);
     }
     g_launches += nl;
     return BBB_OK;
@@ -473,6 +480,29 @@ void bbb_debug_set_mcx_trace(void* dev_ptr) { g_mcx_trace = (long long*)dev_ptr;
 void bbb_debug_set_timeline(void* dev_ptr, int capacity) { g_tl = (long long*)dev_ptr; g_tl_cap = capacity; g_tl_n = 0; }
 int bbb_debug_timeline_count(void) { return g_tl_n; }
 const char* bbb_debug_timeline_name(int k) { return (k >= 0 && k < g_tl_n) ? g_tl_names[k] : ""; }
+/* debug only, host logic only: what bbb_layer_forward_fused launches for this step on a device with n_sm SMs and the
+   given bbb_set_wide_tiles switch.  out[0] kernel (0 conv_s4, 1 gather, 2 tap-GEMM), out[1] tile width BN, out[2] CTAs
+   per SM the GEMM kernel is built for (0 for the gather kernel: its occupancy follows from its shared-memory footprint),
+   out[3] prep kernel (0 weight_prep, 1 conv_s4_prep, 2 tap_prep, 3 tap_prep_conv).  Returns the bbb_fused_supported
+   status; out is written only on BBB_OK. */
+int bbb_debug_fused_config(const bbb_layer_desc* d, int32_t in_layout, int32_t in_pitch, int32_t prev_hw, int32_t out_layout,
+                           int32_t out_pitch, int32_t n_sm, int32_t prefer_wide, int32_t* out) {
+    bbb::Geom g;
+    if (int rc = fused_check(d, g, in_layout, in_pitch, prev_hw, out_layout, out_pitch)) return rc;
+    if (!out || n_sm < 1) return fail(BBB_E_INVALID, "bbb_debug_fused_config: bad arguments");
+    const int kernel = fused_kernel(d, g, in_layout, out_layout);
+    out[0] = kernel;
+    if (kernel == FUSED_KERNEL_CONV_S4) {
+        out[1] = 64; out[2] = 1; out[3] = 1;         // Cout == 64; ~193 KB of shared memory per CTA
+    } else if (kernel == FUSED_KERNEL_GATHER) {
+        out[1] = bbb::TC_BN; out[2] = 0; out[3] = 0;
+    } else {
+        const bbb::TapConfig c = bbb::tap_config(g, bbb::tc_planes(d->variant, d->sample), d->pool_k != 0, prev_hw, n_sm,
+                                                 prefer_wide != 0);
+        out[1] = c.bn; out[2] = c.two_per_sm ? 2 : 1; out[3] = c.prep_conv ? 3 : 2;
+    }
+    return BBB_OK;
+}
 
 const char* bbb_last_error(void) { return g_err; }
 int32_t bbb_abi_version(void) { return BBB_ABI_VERSION; }

@@ -620,25 +620,66 @@ inline bool fused_supported(const Geom& g, int pool) {
     return true;
 }
 
+inline size_t prep2_smem_bytes(int planes, int khw, int r) { return (size_t)planes * khw * prep2_slab(r) * 2; }
+
+// The launch configuration of one tap-GEMM step: launch_fused runs exactly this, and bbb_debug_fused_config reports it.
+struct TapConfig {
+    int bn;            // tile width: 64 or 128 output columns
+    int ng;            // output channels per column group (bn, or bn / 4 with the pool: four pixels per tile)
+    int n_cblk, n_kblk;
+    int two_per_sm;    // BN = 64 with more CTAs than SMs: tap_gemm_kernel<2, 64>, two resident CTAs per SM
+    int prep_conv;     // the prep is tap_prep_conv_kernel (else tap_prep_kernel)
+    int prep_rows;     // tap_prep_conv_kernel: output channels per CTA
+};
+
+inline TapConfig tap_config(const Geom& g, int planes, int pool, int prev_hw, int n_sm, bool prefer_wide) {
+    TapConfig c;
+    // tile width: 128 columns when Cout allows it and the grid still covers most of the machine (operand bytes per MAC,
+    // see tap_gemm_kernel) -- or always when the caller keeps several steps in flight (bbb_set_wide_tiles) -- else 64.  BBB_B200_TAP_BN=64 forces the narrow tile (A/B measurements).
+    const int psets = pool ? (g.OH / 2) * (g.OW / 2) : g.OHW;
+    const int row_tiles = (g.B + TC_BM - 1) / TC_BM;
+    c.bn = 64;
+    {
+        static const int force = [] { const char* e = getenv("BBB_B200_TAP_BN"); return e ? atoi(e) : 0; }();
+        const int ng128 = pool ? 32 : 128;
+        if (g.N % ng128 == 0 && (prefer_wide || (long)psets * (g.N / ng128) * row_tiles >= (long)n_sm * 6 / 10)) c.bn = 128;
+        if (force == 64 || force == 128) c.bn = (force == 128 && g.N % ng128 == 0) ? 128 : 64;
+    }
+    c.ng = pool ? c.bn / 4 : c.bn;
+    c.n_cblk = (g.N + c.ng - 1) / c.ng;
+    c.n_kblk = (g.Cin + 63) / 64;
+    // conv layers: the coalesced prep variant (rows x 64-channel block per CTA); R = rows per CTA, shrunk until the
+    // grid covers the SMs and the staging tile fits 48 KB
+    static const bool prep2_on = [] { const char* e = getenv("BBB_B200_PREP2"); return !(e && e[0] == '0'); }();
+    int R = 8;
+    const int npad = c.n_cblk * c.ng;
+    // <= 26 KB of staging per CTA: the preps run beside the GEMM chain (side streams) and must fit next to its CTAs
+    constexpr size_t kPrepSmem = 26 * 1024;
+    // (smaller CTAs -- >= 4 per SM -- were tried for more loads in flight: the preps then lose the scheduling race against
+    //  the high-priority GEMM chain and the third layer's prep finished at 61 us instead of 21 us: 123 vs 107 us per step)
+    while (R > 2 && ((long)(npad / R) * c.n_kblk < n_sm || prep2_smem_bytes(planes, g.KHW, R) > kPrepSmem)) R >>= 1;
+    c.prep_rows = R;
+    c.prep_conv = prep2_on && g.KHW > 1 && prev_hw == 1 && g.Cin % 64 == 0 && prep2_smem_bytes(planes, g.KHW, R) <= 48 * 1024;
+    // Configurations.  BN = 64: (A) one CTA per SM, stage = 2 K blocks, deep ring; (B) two CTAs per SM (~99 KB each) when
+    // the grid has more CTAs than SMs, so that all tiles run in ONE wave and one CTA's epilogue overlaps the other's main
+    // loop.  BN = 128: one CTA per SM, 64 KB (LRT) / 32 KB K blocks, three stages.
+    const long n_ctas = (long)psets * c.n_cblk * row_tiles;
+    c.two_per_sm = c.bn == 64 && n_ctas > n_sm;
+    return c;
+}
+
 inline cudaError_t launch_fused(FusedArgs a, const void* x, const void* x_sq, cudaStream_t st, int* n_launch, const char** why,
                                 bool do_prep = true, bool do_gemm = true, int n_sm = 148, bool prefer_wide = false) {
     const Geom& g = a.g;
     *n_launch = 0;
     a.planes = tc_planes(a.variant, a.sample);
-    // tile width: 128 columns when Cout allows it and the grid still covers most of the machine (operand bytes per MAC,
-    // see tap_gemm_kernel) -- or always when the caller keeps several steps in flight (bbb_set_wide_tiles) -- else 64.  BBB_B200_TAP_BN=64 forces the narrow tile (A/B measurements).
+    const TapConfig cfg = tap_config(g, a.planes, a.pool, a.prev_hw, n_sm, prefer_wide);
     const int psets = a.pool ? (g.OH / 2) * (g.OW / 2) : g.OHW;
     const int row_tiles = (g.B + TC_BM - 1) / TC_BM;
-    int bn = 64;
-    {
-        static const int force = [] { const char* e = getenv("BBB_B200_TAP_BN"); return e ? atoi(e) : 0; }();
-        const int ng128 = a.pool ? 32 : 128;
-        if (g.N % ng128 == 0 && (prefer_wide || (long)psets * (g.N / ng128) * row_tiles >= (long)n_sm * 6 / 10)) bn = 128;
-        if (force == 64 || force == 128) bn = (force == 128 && g.N % ng128 == 0) ? 128 : 64;
-    }
-    a.ng = a.pool ? bn / 4 : bn;
-    a.n_cblk = (g.N + a.ng - 1) / a.ng;
-    a.n_kblk = (g.Cin + 63) / 64;
+    const int bn = cfg.bn;
+    a.ng = cfg.ng;
+    a.n_cblk = cfg.n_cblk;
+    a.n_kblk = cfg.n_kblk;
     a.taps = g.KHW;
     const bool lrt = a.variant == BBB_VARIANT_LRT;
     a.x = x; a.x_sq = x_sq;
@@ -659,19 +700,9 @@ inline cudaError_t launch_fused(FusedArgs a, const void* x, const void* x_sq, cu
             return true;
         }();
         (void)carve;
-        // conv layers: the coalesced variant (rows x 64-channel block per CTA); R = rows per CTA, shrunk until the
-        // grid covers the SMs and the staging tile fits 48 KB
-        static const bool prep2_on = [] { const char* e = getenv("BBB_B200_PREP2"); return !(e && e[0] == '0'); }();
-        int R = 8;
-        const int npad = a.n_cblk * a.ng;
-        auto need = [&](int r) { return (size_t)a.planes * g.KHW * prep2_slab(r) * 2; };
-        // <= 26 KB of staging per CTA: the preps run beside the GEMM chain (side streams) and must fit next to its CTAs
-        constexpr size_t kPrepSmem = 26 * 1024;
-        // (smaller CTAs -- >= 4 per SM -- were tried for more loads in flight: the preps then lose the scheduling race against
-        //  the high-priority GEMM chain and the third layer's prep finished at 61 us instead of 21 us: 123 vs 107 us per step)
-        while (R > 2 && ((long)(npad / R) * a.n_kblk < n_sm || need(R) > kPrepSmem)) R >>= 1;
-        const bool prep2 = prep2_on && g.KHW > 1 && a.prev_hw == 1 && g.Cin % 64 == 0 && a.taps == g.KHW && need(R) <= 48 * 1024;
-        if (prep2) {
+        const int R = cfg.prep_rows, npad = a.n_cblk * a.ng;
+        const size_t need = prep2_smem_bytes(a.planes, g.KHW, R);
+        if (cfg.prep_conv) {
             static const bool carve2 = [] {
                 const char* e = getenv("BBB_B200_PREP_CARVEOUT");
                 if (e && e[0] == '0') return false;
@@ -682,8 +713,8 @@ inline cudaError_t launch_fused(FusedArgs a, const void* x, const void* x_sq, cu
             (void)carve2;
             int grid2 = (npad / R) * a.n_kblk;
             if (grid2 > 2048) grid2 = 2048;
-            if (lrt) tap_prep_conv_kernel<BBB_VARIANT_LRT><<<grid2, 256, need(R), st>>>(a, R);
-            else     tap_prep_conv_kernel<BBB_VARIANT_BBB><<<grid2, 256, need(R), st>>>(a, R);
+            if (lrt) tap_prep_conv_kernel<BBB_VARIANT_LRT><<<grid2, 256, need, st>>>(a, R);
+            else     tap_prep_conv_kernel<BBB_VARIANT_BBB><<<grid2, 256, need, st>>>(a, R);
         }
         else if (lrt) tap_prep_kernel<BBB_VARIANT_LRT><<<grid, 256, 0, st>>>(a);
         else          tap_prep_kernel<BBB_VARIANT_BBB><<<grid, 256, 0, st>>>(a);
@@ -692,12 +723,8 @@ inline cudaError_t launch_fused(FusedArgs a, const void* x, const void* x_sq, cu
         *n_launch += 1;
     }
     if (!do_gemm) return cudaSuccess;
-    // Configurations.  BN = 64: (A) one CTA per SM, stage = 2 K blocks, deep ring; (B) two CTAs per SM (~99 KB each) when
-    // the grid has more CTAs than SMs, so that all tiles run in ONE wave and one CTA's epilogue overlaps the other's main
-    // loop.  BN = 128: one CTA per SM, 64 KB (LRT) / 32 KB K blocks, three stages.  The LRT noise tile always lives in
-    // tensor memory and is drawn during the main loop.
-    const long n_ctas = (long)psets * a.n_cblk * row_tiles;
-    const bool two_per_sm = bn == 64 && n_ctas > n_sm;
+    // (configurations: see tap_config.)  The LRT noise tile always lives in tensor memory and is drawn during the main loop.
+    const bool two_per_sm = cfg.two_per_sm != 0;
     int stages;
     if (bn == 128)       { stages = 3; a.units = a.planes == 2 ? 1 : 2; }
     else if (two_per_sm) { stages = 2; a.units = a.planes == 2 ? 1 : 2; }

@@ -72,13 +72,14 @@ def test_philox_stream_matches_host_restatement(dev):
 
 
 def _lrt_eps_like(bbb, y, seed, stream, dev):
-    """The activation noise an LRT kernel draws for output y: Philox element index is the
+    """The activation noise an LRT kernel draws for output y (a tensor or a shape): Philox element index is the
     NHWC-flat index of y (include/bbb_b200.h), so fill(numel).view(B,OH,OW,C).permute(0,3,1,2)."""
-    z = bbb.philox_normal(y.numel(), seed, stream, 0, device=dev)
-    if y.dim() == 4:
-        B, C, H, W = y.shape
+    shape = tuple(y.shape) if torch.is_tensor(y) else tuple(y)
+    z = bbb.philox_normal(int(np.prod(shape)), seed, stream, 0, device=dev)
+    if len(shape) == 4:
+        B, C, H, W = shape
         return z.view(B, H, W, C).permute(0, 3, 1, 2).contiguous()
-    return z.view_as(y)
+    return z.view(shape)
 
 
 def test_in_kernel_philox_equals_external_draw(golden_layers, dev):
@@ -384,19 +385,24 @@ def test_fused_equals_unfused_same_philox(dev):
 # --------------------------------------------------------------------------- #
 # backward (SURVEY.md Appendix A) vs torch autograd through the oracle
 # --------------------------------------------------------------------------- #
-def _grad_case(dev, variant, conv, bias, use_philox, math="fp32", tol_y=FP32_TOL, tol_g=1e-4):
+def _grad_case(dev, variant, conv, bias, use_philox, math="fp32", tol_y=FP32_TOL, tol_g=1e-4, shape=None, x_shape=None):
+    """One layer's forward + backward against torch autograd through the oracle.  ``shape``: the layer's constructor
+    arguments, (cin, cout, k, stride, padding) of a conv or (in, out) of a linear layer, and ``x_shape`` its input;
+    by default a 5->7 k3 s2 p1 conv on 6x5x9x8 and a 37->11 linear layer on 9 rows.  Returns the worst gradient error."""
     import pytorch_bayesiancnn_b200 as bbb
     from oracle import bbb_oracle as O
     g = torch.Generator().manual_seed(17)
     if conv:
+        cin, cout, k, s, p = shape or (5, 7, 3, 2, 1)
         cls = bbb.BBB_LRT_Conv2d if variant == "lrt" else bbb.BBB_Conv2d
-        layer = cls(5, 7, 3, stride=2, padding=1, bias=bias, priors=DEF_PRIORS)
-        x = torch.randn(6, 5, 9, 8, generator=g)
-        geom = ((2, 2), (1, 1), (1, 1))
+        layer = cls(cin, cout, k, stride=s, padding=p, bias=bias, priors=DEF_PRIORS)
+        x = torch.randn(x_shape or (6, 5, 9, 8), generator=g)
+        geom = ((s, s), (p, p), (1, 1))
     else:
+        fin, fout = shape or (37, 11)
         cls = bbb.BBB_LRT_Linear if variant == "lrt" else bbb.BBB_Linear
-        layer = cls(37, 11, bias=bias, priors=DEF_PRIORS)
-        x = torch.randn(9, 37, generator=g)
+        layer = cls(fin, fout, bias=bias, priors=DEF_PRIORS)
+        x = torch.randn(x_shape or (9, fin), generator=g)
         geom = None
     layer = layer.to(dev).train()
     layer.set_flag("math", math)
@@ -435,13 +441,16 @@ def _grad_case(dev, variant, conv, bias, use_philox, math="fp32", tol_y=FP32_TOL
         yr = O.bbb_forward(xr, P[0], P[1], P[2], P[3], eps[0], eps[1] if bias else None, geom)
     klr = O.kl_loss(P[0], P[1], P[2], P[3], 0.0, 0.1)
     ((yr * gout).sum() + 0.37 * klr).backward()
-    assert scale_err(y, yr) < tol_y
+    assert scale_err(y, yr) < tol_y, (variant, conv, bias, use_philox, "y", math, scale_err(y, yr))
     got = [xg.grad, layer.W_mu.grad, layer.W_rho.grad] + ([layer.bias_mu.grad, layer.bias_rho.grad] if bias else [])
     ref = [xr.grad, P[0].grad, P[1].grad] + ([P[2].grad, P[3].grad] if bias else [])
+    worst = 0.0
     for name, a, b_ in zip(("x", "W_mu", "W_rho", "bias_mu", "bias_rho"), got, ref):
         assert a is not None, name
         e = scale_err(a, b_)
         assert e < tol_g, (variant, conv, bias, use_philox, name, math, e)
+        worst = max(worst, e)
+    return worst
 
 
 def test_backward_matches_oracle_autograd(dev):
